@@ -24,6 +24,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -354,6 +355,15 @@ def measure_secondary(cfg, dev, rank, world, steps, warmup, tp, batch=BATCH, tag
             "collective": collective}
 
 
+def dump_outputs(d, arrays):
+    """What the last timed step computed, as d/<name>.npy: integers (token ids) as float64, everything else as float32."""
+    os.makedirs(d, exist_ok=True)
+    for name, x in arrays.items():
+        x = x.detach().cpu()
+        x = x.double() if not x.is_floating_point() else x.float()
+        np.save(os.path.join(d, f"{name}.npy"), x.numpy())
+
+
 def bench_c3(a, real_stdout):
     """BASELINE config 3: LServe sparse decode, Llama-3-8B-Instruct-Gradient-1048k shape, 256K context, bs = 1 (1 GPU).
     Harness semantics of scripts/lserve_benchmark (lserve_benchmark.py:79-144): per-token decode latency at a fixed context;
@@ -389,12 +399,14 @@ def bench_c3(a, real_stdout):
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record(); run(n, e2e); t1.record(); torch.cuda.synchronize()
         return t0.elapsed_time(t1)
-    steps = max(interval, (a.steps // interval) * interval)
+    steps = a.steps
     run(max(3, a.warmup))
     sampler = ClockSampler(0); sampler.start()
     ms = timed(steps)
     clocks = sampler.stop()
     ms_e2e = timed(steps, e2e=True)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"next_tokens": graphs.out})
 
     def one(sel, n=8):
         torch.cuda.synchronize()
@@ -457,6 +469,10 @@ def main():
                          "exchange after o_proj and after down_proj; same global batch of 64 -> strong scaling), dp = one "
                          "bs=64 replica per GPU (weak scaling, no data-path collective).  auto = tp as the headline, with the "
                          "dp measurement added under \"dp\".")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (sampled next tokens; c2 also the final "
+                         "hidden state of every sequence) as DIR/<name>.npy; the inputs are seeded, so runs with the same "
+                         "arguments can be compared output for output")
     a = ap.parse_args()
     # Keep stdout clean for the ONE JSON line: libraries (NCCL banner, warnings) print to fd 1 in worker processes.
     real_stdout = os.fdopen(os.dup(1), "w")
@@ -616,6 +632,12 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     run_steps(3, e2e=True)
     ms_e2e = timed(a.steps, e2e=True)
+    if a.dump_outputs and rank == 0:
+        h, delta = model.last_decode_state
+        outs = {"next_tokens": out_buf}
+        if torch.is_tensor(delta):   # hidden state after the last layer, before the final norm
+            outs["final_hidden"] = h.float() + delta.float()
+        dump_outputs(a.dump_outputs, outs)
 
     value = BATCH * replicas * a.steps / (ms / 1e3)
     e2e_value = BATCH * replicas * a.steps / (ms_e2e / 1e3)

@@ -2,6 +2,7 @@
 import importlib.machinery
 import importlib.util
 import os
+import zlib
 
 import numpy as np
 import torch
@@ -31,6 +32,105 @@ def ref_module(name):
         loader.exec_module(mod)
     _ref_cache[name] = mod
     return mod
+
+
+GOLDEN_REF = os.path.join(ROOT, "tests", "golden", "ref_kernels.npz")
+RECORD_REF = os.environ.get("OB_RECORD_REF_GOLDEN")   # path of an .npz that live reference runs are recorded into
+SAMPLE = 1024
+
+
+class RefOutputs:
+    """What the reference's own kernel computed for one test case.  Live (oracle/_ref present): the full arrays.  Otherwise
+    the record in tests/golden/ref_kernels.npz: per array a fixed seeded sample of SAMPLE elements (all of them when the
+    array is smaller), its shape and its largest magnitude, plus any statistic the test derived from the full arrays."""
+
+    def __init__(self, case, arrays, bases=None):
+        self.case, self.arrays, self.bases = case, arrays, bases or {}
+        self.golden = None
+        if arrays is None:
+            assert os.path.exists(GOLDEN_REF), f"{GOLDEN_REF} missing"
+            self.golden = np.load(GOLDEN_REF)
+            assert any(k.startswith(case + "|") for k in self.golden.files), f"no recorded reference outputs for {case}"
+
+    def _key(self, name, what):
+        return f"{self.case}|{name}|{what}"
+
+    def _g(self, name, what):
+        k = self._key(name, what)
+        assert k in self.golden.files, f"{k} not recorded in {GOLDEN_REF}"
+        return self.golden[k]
+
+    def pair(self, name, ours):
+        """(ours, reference) as flat arrays over the same elements: all of them live, the recorded sample otherwise."""
+        ours = ours.cpu().numpy() if torch.is_tensor(ours) else np.asarray(ours)
+        if self.golden is None:
+            ref = self.arrays[name]
+            assert ours.shape == ref.shape
+            return ours.reshape(-1), ref.reshape(-1)
+        assert tuple(ours.shape) == tuple(self._g(name, "shape")), f"{name}: shape {ours.shape}"
+        if self._key(name, "didx") in self.golden.files:   # the whole array: its input state plus the recorded changes
+            ref = np.array(self.bases[name]).reshape(-1)
+            ref[self._g(name, "didx")] = self._g(name, "dval")
+            return ours.reshape(-1), ref
+        v = self._g(name, "v")
+        if v.size == ours.size:                             # recorded whole
+            return ours.reshape(-1), v
+        return ours.reshape(-1)[_sample_index(self.case, name, ours.size)], v
+
+    def absmax(self, name):
+        if self.golden is None:
+            return float(np.abs(self.arrays[name].astype(np.float64)).max())
+        return float(self._g(name, "absmax"))
+
+    def stat(self, name, fn):
+        """fn(full reference arrays) -> float, computed live (and recorded) or read from the record."""
+        if self.golden is None:
+            v = float(fn(self.arrays))
+            if RECORD_REF:
+                _record({self._key(name, "stat"): np.float64(v)})
+            return v
+        return float(self._g(name, "stat"))
+
+
+def _sample_index(case, name, size):
+    if size <= SAMPLE:
+        return np.arange(size)
+    rng = np.random.default_rng(zlib.crc32(f"{case}|{name}".encode()))
+    return np.sort(rng.choice(size, SAMPLE, replace=False))
+
+
+def _record(entries):
+    old = dict(np.load(RECORD_REF)) if os.path.exists(RECORD_REF) else {}
+    old.update(entries)
+    np.savez_compressed(RECORD_REF, **old)
+
+
+def reference_outputs(case, live, run, bases=None, whole=()):
+    """Outputs of the reference's own kernels for test case `case`: run() -> {name: np.ndarray} when `live` (the
+    oracle/_ref modules the case needs are present; recorded when OB_RECORD_REF_GOLDEN is set), the committed record
+    otherwise.  A case without a record fails: the comparison with the reference is never skipped.
+    bases: {name: the array's state before the kernel ran} for arrays the kernel changes in a few places (KV page pools
+    it appends one token to): those are recorded as their changed elements and replayed whole.  whole: names of small
+    arrays recorded in full rather than sampled."""
+    bases = {k: (v.cpu().numpy() if torch.is_tensor(v) else np.asarray(v)) for k, v in (bases or {}).items()}
+    if not live:
+        return RefOutputs(case, None, bases)
+    arrays = {k: (v.cpu().numpy() if torch.is_tensor(v) else np.asarray(v)) for k, v in run().items()}
+    if RECORD_REF:
+        rec = {}
+        for name, a in arrays.items():
+            k = f"{case}|{name}|"
+            if name in bases:
+                d = np.flatnonzero(a.reshape(-1) != bases[name].reshape(-1))
+                rec[k + "didx"], rec[k + "dval"] = d, a.reshape(-1)[d]
+            elif name in whole:
+                rec[k + "v"] = a.reshape(-1)
+            else:
+                rec[k + "v"] = a.reshape(-1)[_sample_index(case, name, a.size)]
+            rec[k + "shape"] = np.asarray(a.shape, np.int64)
+            rec[k + "absmax"] = np.float64(np.abs(a.astype(np.float64)).max()) if a.size else np.float64(0)
+        _record(rec)
+    return RefOutputs(case, arrays)
 
 
 def make_gemm_inputs(M, N, K, seed, per_group=False):

@@ -1,5 +1,5 @@
 """-m gpu: static per-tensor INT8 KV pages (SURVEY.md section 8 row f4) -- fused_attention_per_tensor_{dense,sparse} vs
-oracle/kv8.py and, when oracle/_ref ships it, vs the reference's own fused_attention_per_tensor_dense kernels.
+oracle/kv8.py and vs the reference's own fused_attention_per_tensor_dense kernels (oracle/_ref, or their recorded outputs).
 
 Tolerance: the stored codes are consumed exactly (int8 -> fp16 is exact, fp32 accumulation), so the distance to the
 EXACT-arithmetic oracle is bounded by the fp16 probability rounding: 2e-3 of the output scale, as for KV4
@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.gpu_util import device_tables, qkv_views, ref_module, t
+from tests.gpu_util import device_tables, qkv_views, ref_module, reference_outputs, t
 
 pytestmark = pytest.mark.gpu
 TOL_EXACT = 2e-3
@@ -222,8 +222,6 @@ def test_kv8_vs_reference_kernels():
     ours; decode output within 3e-3 of the output scale of ours (the reference rounds dequantised values and probabilities
     to fp16; ours is closer to exact)."""
     ref = ref_module("fused_attention_per_tensor_dense")
-    if ref is None:
-        pytest.skip("oracle/_ref/fused_attention_per_tensor_dense not shipped")
     from omniserve_b200.backend import fused_attention_per_tensor_dense as ours
     from oracle import kv8
     rng = np.random.default_rng(17)
@@ -247,28 +245,38 @@ def test_kv8_vs_reference_kernels():
     sl = t(np.asarray(lens, np.int32))
     cu = t(np.concatenate([[0], np.cumsum(lens)]).astype(np.int32))
     pad = ours.compute_padding_offsets(cu, max(lens), T)
-    outs = []
-    for mod, (cache, btab, kp, vp, ptr) in zip((ref, ours), pools):
+    db = pools[0][0].data_bytes
+
+    def prefill(mod, kp, vp, ptr):
         x = t(qkv)
         mod.apply_bias_rope_update_kv_cache(x, t(soq), sl, None, pad, ptr, None, flags, rank, Hq, Hkv, max(lens), 64, Hkv * Dh, 0,
                                             0, 0, 0, 0, Hkv, 0, 128, BASE, 1.0, 8192, True, False, False)   # max_positions != 0
         torch.cuda.synchronize()
-        outs.append((x.cpu().numpy(), kp.cpu().numpy().copy(), vp.cpu().numpy().copy()))
-    np.testing.assert_array_equal(outs[0][2][:, : pools[0][0].data_bytes], outs[1][2][:, : pools[0][0].data_bytes])
-    dk = np.abs(outs[0][1][:, : pools[0][0].data_bytes].view(np.int8).astype(np.int32) -
-                outs[1][1][:, : pools[0][0].data_bytes].view(np.int8).astype(np.int32))
-    assert dk.max() <= 1 and (dk != 0).mean() < 1e-3
+        return kp.cpu().numpy().copy(), vp.cpu().numpy().copy()
     q = rng.standard_normal((B, Hq, Dh)).astype(np.float16)
     k = rng.standard_normal((B, Hkv, Dh)).astype(np.float16)
     v = rng.standard_normal((B, Hkv, Dh)).astype(np.float16)
     lens1 = t(np.asarray([l + 1 for l in lens], np.int32))
-    res = []
-    for mod, (cache, btab, kp, vp, ptr) in zip((ref, ours), pools):
-        kp.copy_(torch.from_numpy(outs[1][1]).cuda()); vp.copy_(torch.from_numpy(outs[1][2]).cuda())   # same pages for both
+
+    def decode(mod, kp, vp, ptr, pages):
+        kp.copy_(torch.from_numpy(pages[0]).cuda()); vp.copy_(torch.from_numpy(pages[1]).cuda())   # same pages for both
         _, tq, tk, tv = qkv_views(q, k, v)
         o = mod.single_query_attention(tq, tk, tv, t(sqo), t(soq), ptr, None, flags, rank, lens1, None, 4096, 64, Hkv * Dh, 0, 0, 0,
                                        0, 0, Hkv, 0, max(lens), 128, BASE, 1.0, True, False, False, 2048)
         torch.cuda.synchronize()
-        res.append(o.cpu().numpy().astype(np.float32))
-    sc = np.abs(res[1]).max()
-    assert np.abs(res[0] - res[1]).max() <= 3e-3 * sc, np.abs(res[0] - res[1]).max() / sc
+        return o.cpu().numpy().astype(np.float32)
+    mine = prefill(ours, *pools[1][2:])
+
+    def run():
+        kp_ref, vp_ref = prefill(ref, *pools[0][2:])
+        return {"k_data": kp_ref[:, :db], "v_data": vp_ref[:, :db], "out": decode(ref, *pools[0][2:], mine)}
+    r = reference_outputs("kv8_300_77_1030", ref is not None, run)
+    a, b = r.pair("v_data", mine[1][:, :db])
+    np.testing.assert_array_equal(a, b)
+    a, b = r.pair("k_data", mine[0][:, :db])
+    dk = np.abs(a.view(np.int8).astype(np.int32) - b.view(np.int8).astype(np.int32))
+    assert dk.max() <= 1 and (dk != 0).mean() < 1e-3
+    got = decode(ours, *pools[1][2:], mine)
+    sc = np.abs(got).max()
+    a, b = r.pair("out", got)
+    assert np.abs(a - b).max() <= 3e-3 * sc, np.abs(a - b).max() / sc

@@ -1,11 +1,11 @@
 """-m gpu: LServe page statistics (a11), page selector (a9) and the dynamic-sparse decode loop built from them,
-through the C ABI, against the oracle and -- when oracle/_ref was shipped -- the reference's own kernels rebuilt
-for sm_100 (sparse_utils/ContextPool, sparse_utils/KVPageSelector)."""
+through the C ABI, against the oracle and the reference's own kernels rebuilt for sm_100 (oracle/_ref, or their
+recorded outputs in tests/golden/ref_kernels.npz) (sparse_utils/ContextPool, sparse_utils/KVPageSelector)."""
 import numpy as np
 import pytest
 import torch
 
-from tests.gpu_util import assert_k_pool_equal, qkv_views, ref_module, t
+from tests.gpu_util import assert_k_pool_equal, qkv_views, ref_module, reference_outputs, t
 
 pytestmark = pytest.mark.gpu
 
@@ -49,17 +49,19 @@ def test_paged_min_max_pool_bit_exact(lens):
     kv4.paged_min_max_pool(cache, bt, keys, lens, 16, pooling_heads_idx=idx)
     np.testing.assert_array_equal(kpool.cpu().numpy(), cache.k_pool)
     ref = ref_module("fused_attention_ctx_pool")
-    if ref is not None:
+
+    def run():
         kpool2, _, ptrs2 = _ptrs(cache, bt)
         kpool2.view(torch.uint8)[:] = 7
-        kp_mine = kpool.clone()
         ref.paged_min_max_pool(t(keys), ptrs2, t(cu), t(idx), max(lens), 16, 64, 2 * 64, True)
         torch.cuda.synchronize()
-        # compare only the statistics the reference wrote (its pool was filled with 7s first)
-        a = kpool2.cpu().numpy()
-        wrote = a != 7
-        np.testing.assert_array_equal(a[wrote], kp_mine.cpu().numpy()[wrote])
-        assert wrote.sum() >= 2 * 2 * 256 * sum((l + 15) // 16 for l in lens) * 0.95
+        return {"k_pool": kpool2}
+    r = reference_outputs(f"ctx_pool_{'_'.join(map(str, lens))}", ref is not None, run)
+    # compare only the statistics the reference wrote (its pool was filled with 7s first)
+    mine, a = r.pair("k_pool", kpool)
+    wrote = a != 7
+    np.testing.assert_array_equal(a[wrote], mine[wrote])
+    assert r.stat("bytes_written", lambda ref_: (ref_["k_pool"] != 7).sum()) >= 2 * 2 * 256 * sum((l + 15) // 16 for l in lens) * 0.95
 
 
 def _selector_args(tq, tk, tv, ptrs, flags, rank, lens_t, Hkv_r, timestep):
@@ -115,8 +117,7 @@ def test_page_selector_scores_vs_reference_kernel(lens, group, tmp_path):
     from oracle import kv4
     from tests.gpu_util import REF_DIR, ROOT
     shim = os.path.join(ROOT, "oracle", "_ref", "libref_launch_shim.so")
-    if not os.path.exists(os.path.join(REF_DIR, "fused_attention_selector.so")) or not os.path.exists(shim):
-        pytest.skip("oracle/_ref selector module or launch shim not shipped")
+    live = os.path.exists(os.path.join(REF_DIR, "fused_attention_selector.so")) and os.path.exists(shim)
     Hkv = 2
     Hq = Hkv * group
     flags_np, rank_np = np.array([1, 1], np.int32), np.array([1, 0], np.int32)
@@ -128,21 +129,22 @@ def test_page_selector_scores_vs_reference_kernel(lens, group, tmp_path):
     k = rng.standard_normal((len(lens), Hkv, 128)).astype(np.float16)
     v = rng.standard_normal((len(lens), Hkv, 128)).astype(np.float16)
     timestep = max(lens) - 1
-    inp, outp = str(tmp_path / "in.npz"), str(tmp_path / "out.npz")
-    np.savez(inp, k_pool=cache.k_pool, bt=bt, k_page_bytes=cache.k_page_bytes, q=q, k=k, v=v, flags=flags_np, rank=rank_np,
-             lens=np.asarray(lens, np.int32), timestep=timestep, Hr=Hr)
-    env = dict(os.environ, LD_PRELOAD=shim)
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "ref_selector_worker.py"), inp, outp], env=env,
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, f"reference selector failed even with the shared-memory shim:\n{r.stdout[-1500:]}\n{r.stderr[-1500:]}"
-    ref_out = np.load(outp)["out"]
+    def run():
+        inp, outp = str(tmp_path / "in.npz"), str(tmp_path / "out.npz")
+        np.savez(inp, k_pool=cache.k_pool, bt=bt, k_page_bytes=cache.k_page_bytes, q=q, k=k, v=v, flags=flags_np, rank=rank_np,
+                 lens=np.asarray(lens, np.int32), timestep=timestep, Hr=Hr)
+        env = dict(os.environ, LD_PRELOAD=shim)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "ref_selector_worker.py"), inp, outp], env=env,
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, f"reference selector failed even with the shared-memory shim:\n{r.stdout[-1500:]}\n{r.stderr[-1500:]}"
+        return {"out": np.load(outp)["out"]}
+    rec = reference_outputs(f"selector_{'_'.join(map(str, lens))}_g{group}", live, run)
     _, tq, tk, tv = qkv_views(q, k, v)
     kpool, _, ptrs = _ptrs(cache, bt)
     out = op.single_query_page_selector(*_selector_args(tq, tk, tv, ptrs, t(flags_np), t(rank_np), t(np.asarray(lens, np.int32)),
                                                         Hr, timestep))
     torch.cuda.synchronize()
-    got = out.cpu().numpy()
-    assert got.shape == ref_out.shape
+    got, ref_out = rec.pair("out", out)
     g32, r32 = got.astype(np.float32), ref_out.astype(np.float32)
     # the reference rotates q with fast-math sin/cos (ours: accurate sincosf), so a few scores differ in the last bits
     print(f"\nselector vs reference kernel lens={lens} group={group}: identical={np.mean(got == ref_out):.4f} "

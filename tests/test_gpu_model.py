@@ -54,26 +54,34 @@ def test_fused_silu_quant_equals_two_kernel_chain():
 
 
 def test_whole_stack_vs_reference_kernels():
-    """Same weights, same prompts through the reference's rebuilt kernels (oracle/_ref) and ours."""
-    from tests.gpu_util import ref_module
+    """Same weights, same prompts through the reference's rebuilt kernels (oracle/_ref, or their recorded outputs) and
+    ours."""
+    from tests.gpu_util import ref_module, reference_outputs
     from omniserve_b200.model import Ops
-    if ref_module("qgemm_w4a8_per_chn") is None:
-        pytest.skip("oracle/_ref not shipped")
     cfg, ours = _mk(fuse=False)
-    cfg, ref = _mk(ops=Ops(ref_module), fuse=False)
     toks, lens = _prompts(cfg)
-    a, b = ours.prefill(toks, lens), ref.prefill(toks, lens)
-    ha, hb = ours.last_hidden.float(), ref.last_hidden.float()
-    assert (ha - hb).abs().max() <= 2e-2 * hb.abs().max()      # two layers of fp16 / int8-rounding drift
+    a = ours.prefill(toks, lens)
+
+    def run():
+        cfg, ref = _mk(ops=Ops(ref_module), fuse=False)
+        ref.prefill(toks, lens)
+        res = {"prefill_hidden": ref.last_hidden.float(), "v_pages_layer0": ref.kv.v_pools[0].clone()}   # before decode appends
+        ref.prepare_decode()
+        ref.decode_step(a.clone(), 192)
+        res["decode_hidden"] = ref.last_decode_state[0].float() + ref.last_decode_state[1].float()
+        return res
+    r = reference_outputs("model_tiny_prefill_decode", ref_module("qgemm_w4a8_per_chn") is not None, run,
+                          whole=("v_pages_layer0",))
+    x, y = r.pair("prefill_hidden", ours.last_hidden.float())
+    assert np.abs(x - y).max() <= 2e-2 * r.absmax("prefill_hidden")      # two layers of fp16 / int8-rounding drift
     # V pages byte-identical would need identical hidden states; compare the first layer's pages instead
-    assert (ours.kv.v_pools[0] != ref.kv.v_pools[0]).float().mean() < 2e-3
-    ours.prepare_decode(); ref.prepare_decode()
-    t = a.clone()
-    o = ours.decode_step(t, 192)
-    ho = (ours.last_decode_state[0].float() + ours.last_decode_state[1].float()).clone()
-    r = ref.decode_step(t, 192)
-    hr = ref.last_decode_state[0].float() + ref.last_decode_state[1].float()
-    assert (ho - hr).abs().max() <= 3e-2 * hr.abs().max()
+    x, y = r.pair("v_pages_layer0", ours.kv.v_pools[0])
+    assert (x != y).mean() < 2e-3
+    ours.prepare_decode()
+    ours.decode_step(a.clone(), 192)
+    ho = ours.last_decode_state[0].float() + ours.last_decode_state[1].float()
+    x, y = r.pair("decode_hidden", ho)
+    assert np.abs(x - y).max() <= 3e-2 * r.absmax("decode_hidden")
 
 
 def test_reference_op_chain_equals_fused_production_path_bit_for_bit():

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.gpu_util import device_tables, make_kv_case, qkv_views, ref_module, t
+from tests.gpu_util import device_tables, make_kv_case, qkv_views, ref_module, reference_outputs, t
 
 pytestmark = pytest.mark.gpu
 
@@ -106,30 +106,29 @@ def test_dense_attention_not_worse_than_reference_kernel(lens, record_property):
     q.k partial sums, fp16 probabilities) put it ~1e-3 from exact arithmetic; both errors are measured here."""
     from oracle import kv4
     from omniserve_b200.backend import fused_attention_pure_dense as ours
-    ref = ref_module("fused_attention_pure_dense")
     B, Hq, Hkv = len(lens), 32, 8
     cache, bt, q, k, v = make_kv_case(B, Hq, Hkv, lens, seed=sum(lens) + 5)
-    outs = {}
-    for name, impl in (("ref", ref), ("ours", ours)):
-        if impl is None:
-            continue
+
+    def call(impl):
         kpool, vpool, ptrs = device_tables(cache, bt)
         _, tq, tk, tv = qkv_views(q, k, v)
         o = impl.single_query_attention(tq, tk, tv, ptrs, t(np.asarray(lens, np.int32)), None, 2048, 64, Hkv * 64, max(lens),
                                         128, 500000.0, True, True, True)
         torch.cuda.synchronize()
-        outs[name] = o.cpu().numpy()
+        return o.cpu().numpy()
+    live = ref_module("fused_attention_pure_dense") is not None
+    r = reference_outputs(f"parity_attention_{'_'.join(map(str, lens))}", live,
+                          lambda: {"out": call(ref_module("fused_attention_pure_dense"))})
+    got = call(ours)
     exact = kv4.decode_attention(q, k, v, cache, bt, lens, 128, 500000.0, mimic=False, append=False)
-    e_ours = _err(outs["ours"], exact)
+    e_ours = _err(got, exact)
     record_property("err_ours", e_ours)
-    print(f"\nattention lens={lens}: |ours-exact|={e_ours:.3e}", end="")
-    if "ref" in outs:
-        e_ref = _err(outs["ref"], exact)
-        record_property("err_ref", e_ref)
-        print(f" |ref-exact|={e_ref:.3e} |ours-ref|={_err(outs['ours'], outs['ref']):.3e}")
-        assert e_ours <= max(e_ref, NORTH_STAR)
-    else:
-        assert e_ours <= 2e-3
+    e_ref = r.stat("err_vs_exact", lambda ref: _err(ref["out"], exact))
+    record_property("err_ref", e_ref)
+    a, b = r.pair("out", got)
+    print(f"\nattention lens={lens}: |ours-exact|={e_ours:.3e} |ref-exact|={e_ref:.3e} "
+          f"|ours-ref|={np.abs(a.astype(np.float32) - b.astype(np.float32)).max() / np.abs(exact).max():.3e}")
+    assert e_ours <= max(e_ref, NORTH_STAR)
 
 
 def test_prefill_write_then_decode_without_host_sync():

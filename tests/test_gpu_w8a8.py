@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.gpu_util import ref_module, t
+from tests.gpu_util import ref_module, reference_outputs, t
 
 pytestmark = pytest.mark.gpu
 
@@ -36,12 +36,16 @@ def test_w8a8_gemm_vs_oracle_and_reference_kernel(M, N, K):
     assert np.abs(g32 - r32).max() <= 1e-3 * np.abs(r32).max()
     assert (got == ref).mean() > 0.999
     rm = ref_module("qgemm_w8a8")
-    if rm is not None and N % (256 if M > 128 else 64) == 0:   # the reference tiles N by 64 (M <= 128) / 256 without masking
-        o2 = torch.zeros((M, N), dtype=torch.float16, device="cuda")
-        rm.w8a8_gemm_forward_cuda(*args, o2)
-        torch.cuda.synchronize()
-        assert (o2.float() - out.float()).abs().max() <= 1e-3 * o2.float().abs().max()
-        assert (o2 == out).float().mean() > 0.999
+    if N % (256 if M > 128 else 64) == 0:   # the reference tiles N by 64 (M <= 128) / 256 without masking
+        def run():
+            o2 = torch.zeros((M, N), dtype=torch.float16, device="cuda")
+            rm.w8a8_gemm_forward_cuda(*args, o2)
+            torch.cuda.synchronize()
+            return {"out": o2}
+        r = reference_outputs(f"w8a8_{M}x{N}x{K}", rm is not None, run)
+        a, b = r.pair("out", got)
+        assert np.abs(a.astype(np.float32) - b.astype(np.float32)).max() <= 1e-3 * r.absmax("out")
+        assert (a == b).mean() > 0.999
 
 
 def test_w8a8_int32_accumulators_exact():
