@@ -239,6 +239,32 @@ int ob_kv4_page_selector(const ob_page_selector_args* args, void* stream);
 int ob_kv4_page_topk(const void* scores, int32_t* out, int rows, int pitch_sub_chunks, int sub_chunks_per_page,
                      int total_pages, int k_out, void* stream);
 
+/* ---- block_sparse_attn.token_streaming_attn_func for LServe's streaming heads (caller: ctx_attn_func.py:62-73; masks
+ * ctx_attn_init.py:11-52).  fp16 causal prefill attention over variable-length sequences with the token-streaming mask:
+ * query position i of a sequence attends key position j  iff  j <= i  and  (j < sink  or  i - j < local), which is the
+ * window the streaming-head decode attention keeps (the sink plus the last `local` tokens, the current one included).
+ * q [T, Hq, 128], k / v [T, Hkv, 128]: strided views (head stride 128, token strides below, e.g. into the qkv activation;
+ * k / v 16-byte aligned, token strides multiples of 8).  out: fp16 [T, Hq, 128] contiguous; only the q-heads of the
+ * kv heads listed in kv_heads are written.  cu_seqlens, kv_heads, sink, local are HOST arrays.  Hq / Hkv must divide
+ * 128; at most 64 kv heads per call; sink >= 0, local >= 1.  Deterministic (no atomics). */
+typedef struct ob_streaming_prefill_args {
+  const void* q; const void* k; const void* v;
+  long long q_row_stride, k_row_stride, v_row_stride; /* elements */
+  void* out;
+  const int32_t* cu_seqlens;                          /* HOST [batch + 1] */
+  int batch, num_tokens, num_heads, num_kv_heads, head_dim;
+  int num_compute_kv_heads;
+  const int32_t* kv_heads;                            /* HOST [num_compute_kv_heads] */
+  const int32_t* sink; const int32_t* local;          /* HOST [num_compute_kv_heads]: the (sink, local) of each kv group */
+} ob_streaming_prefill_args;
+int ob_token_streaming_prefill_attention(const ob_streaming_prefill_args* args, void* stream);
+/* Host-only (no CUDA call, usable without a GPU): the launch plan of the call above.  out[0] = launches, out[1] / out[2] =
+ * grid x / y of launch `launch`, out[3] = sequence, out[4] / out[5] = first / last query position (within the sequence) of
+ * CTA (cta_x, cta_y), out[6] = its kv head, out[7] = number of 64-key tiles it visits, whose indices are written to
+ * key_tiles (at most max_key_tiles).  Device pointers in args may be NULL. */
+int ob_debug_streaming_prefill_plan(const ob_streaming_prefill_args* args, int launch, int cta_x, int cta_y, int* out,
+                                    int* key_tiles, int max_key_tiles);
+
 #ifdef __cplusplus
 }
 #endif

@@ -73,6 +73,17 @@ class PageSelectorArgs(C.Structure):
     ]
 
 
+class StreamingPrefillArgs(C.Structure):
+    _fields_ = [
+        ("q", c_p), ("k", c_p), ("v", c_p),
+        ("q_row_stride", c_ll), ("k_row_stride", c_ll), ("v_row_stride", c_ll),
+        ("out", c_p), ("cu_seqlens", c_p),
+        ("batch", c_i), ("num_tokens", c_i), ("num_heads", c_i), ("num_kv_heads", c_i), ("head_dim", c_i),
+        ("num_compute_kv_heads", c_i),
+        ("kv_heads", c_p), ("sink", c_p), ("local", c_p),
+    ]
+
+
 _SIGS = {
     "ob_version": ([], c_i),
     "ob_error_string": ([c_i], C.c_char_p),
@@ -102,6 +113,8 @@ _SIGS = {
     "ob_paged_min_max_pool": ([c_p] * 4 + [c_ll] * 2 + [c_i] * 9 + [c_p], c_i),
     "ob_kv4_page_topk": ([c_p] * 2 + [c_i] * 5 + [c_p], c_i),
     "ob_kv4_page_selector": ([C.POINTER(PageSelectorArgs), c_p], c_i),
+    "ob_token_streaming_prefill_attention": ([C.POINTER(StreamingPrefillArgs), c_p], c_i),
+    "ob_debug_streaming_prefill_plan": ([C.POINTER(StreamingPrefillArgs)] + [c_i] * 3 + [c_p] * 2 + [c_i], c_i),
 }
 EXPORTS = tuple(_SIGS)
 

@@ -2,6 +2,7 @@
 #include "../../include/omniserve_b200.h"
 #include "kv4_attention.h"
 #include "lserve_ops.h"
+#include "prefill_attention.h"
 #include "small_ops.h"
 #include "w4a8_gemm.h"
 
@@ -267,6 +268,28 @@ int ob_kv4_page_selector(const ob_page_selector_args* x, void* stream) {
   a.tokens_per_sub_chunk = x->tokens_per_sub_chunk;
   a.hidden_dim_per_retrieval_token = x->hidden_dim_per_retrieval_token;
   return page_selector_run(a, ST(stream));
+}
+
+static StreamingPrefillArgs to_streaming(const ob_streaming_prefill_args* x) {
+  StreamingPrefillArgs a{};
+  a.q = H(x->q); a.k = H(x->k); a.v = H(x->v);
+  a.q_row_stride = x->q_row_stride; a.k_row_stride = x->k_row_stride; a.v_row_stride = x->v_row_stride;
+  a.out = HM(x->out); a.cu_seqlens_host = x->cu_seqlens;
+  a.B = x->batch; a.T = x->num_tokens; a.Hq = x->num_heads; a.Hkv = x->num_kv_heads; a.head_dim = x->head_dim;
+  a.num_compute_heads = x->num_compute_kv_heads; a.kv_heads_host = x->kv_heads;
+  a.sink_host = x->sink; a.local_host = x->local;
+  return a;
+}
+
+int ob_token_streaming_prefill_attention(const ob_streaming_prefill_args* x, void* stream) {
+  if (!x) return OB_ERR_ARG;
+  return streaming_prefill_run(to_streaming(x), ST(stream));
+}
+
+int ob_debug_streaming_prefill_plan(const ob_streaming_prefill_args* x, int launch, int cta_x, int cta_y, int* out,
+                                    int* key_tiles, int max_key_tiles) {
+  if (!x) return OB_ERR_ARG;
+  return streaming_prefill_plan(to_streaming(x), launch, cta_x, cta_y, out, key_tiles, max_key_tiles);
 }
 
 int ob_kv4_page_topk(const void* scores, int32_t* out, int rows, int pitch_sub_chunks, int sub_chunks_per_page,
