@@ -265,6 +265,47 @@ int ob_token_streaming_prefill_attention(const ob_streaming_prefill_args* args, 
 int ob_debug_streaming_prefill_plan(const ob_streaming_prefill_args* args, int launch, int cta_x, int cta_y, int* out,
                                     int* key_tiles, int max_key_tiles);
 
+/* ==== Mixture-of-experts block (Mixtral).  The reference's MixtralSparseMoeBlockOurs.forward calls these ops but never released
+ * them (omniserve/modeling/models/mixtral_w4a8_unpad.py:300-395, raises NotImplementedError at :309); oracle/moe.py pins the
+ * semantics.  All are deterministic and row-independent; E <= 64 experts, 1 <= k <= min(E, 8) experts per token. */
+
+/* ---- router logits (`router_logits = self.gate(hidden_states).float()`, :277,305): logits fp32 [T, E] = fp16-rounded
+ * sum_h x[t,h] * gate_weight[e,h]; x fp16 [T, H] (the post_attention_layernorm output), gate_weight fp16 [E, H].  H % 8 == 0. */
+int ob_moe_router_logits(const void* x, const void* gate_weight, float* logits, int T, int H, int E, void* stream);
+
+/* ---- moe_helpers.moe_topk_gating_softmax (:315) + the expert histogram the caller builds with torch.bincount (:320), on the
+ * device in one CTA: p = softmax(logits) (fp32), the k most probable experts (ties -> lower index; slots in descending p),
+ * routing_weights fp32 [T, k] = p_sel / sum(p_sel); expert_indices int32 [T*k] token-major; rows sorted by expert, stably by
+ * (token, slot): permuted_loc_to_unpermuted_loc int32 [T*k] (value t*k + j); expert_offsets int32 [E+1] (cumulative). */
+int ob_moe_topk_sort(const float* logits, float* routing_weights, int32_t* expert_indices, int32_t* permuted_loc_to_unpermuted_loc,
+                     int32_t* expert_offsets, int T, int E, int k, void* stream);
+
+/* ---- moe_helpers.moe_expand_inputs_and_scales (:345): row r of q_out / ssums_out / scales_out = row (perm[r] / k) of the
+ * per-token INT8 activations (invoke_quant_fuse_sum output, :334) / sums / scales; unpermuted_loc_to_permuted_loc[perm[r]] = r.
+ * q_input_ssums / ssums_out may both be NULL.  H % 16 == 0. */
+int ob_moe_expand(const int8_t* q_hidden_states, const void* q_input_ssums, const void* q_input_scales,
+                  const int32_t* permuted_loc_to_unpermuted_loc, int8_t* q_out, void* ssums_out, void* scales_out,
+                  int32_t* unpermuted_loc_to_permuted_loc, int T, int k, int H, void* stream);
+
+/* ---- moe_helpers.moe_finalize_routing (:388): out fp16 [T, H] = fp16(sum_j routing_weights[t,j] * q_w2_out[inv[t*k+j]]),
+ * fp32, j ascending; q_w2_out fp16 [T*k, ldy]. */
+int ob_moe_finalize(const void* q_w2_out, const float* routing_weights, const int32_t* unpermuted_loc_to_permuted_loc, void* out,
+                    int T, int k, int H, int ldy, void* stream);
+
+/* ---- the w1_w3 / w2 grouped GEMMs of the block (:354,382) with the expert row ranges in DEVICE memory: as ob_w4a8_moe_gemm, but
+ * expert e owns rows [expert_offsets[e], expert_offsets[e+1]) of the total_rows rows (the ob_moe_topk_sort output) and gets at
+ * most 64 of them -- which holds whenever the layer has <= 64 tokens, since a token routes to distinct experts.  No host
+ * read-back: capturable in a CUDA graph.  Rows are clamped to [0, total_rows] and cut at 64, so a malformed table cannot
+ * address outside in_feats / out.  num_experts <= 64. */
+int ob_w4a8_moe_gemm_dev(const int8_t* in_feats, const int8_t* kernel, const void* wscales, const void* ascales,
+                         const void* w_szs, const void* a_ssums, void* out_feats, const int32_t* expert_offsets, int num_experts,
+                         int total_rows, int N, int K, int ldc, void* stream);
+/* Host-only (no CUDA call, usable without a GPU): the schedule of the call above on a device with `sms` SMs for the HOST table
+ * offsets_host [E+1].  grid / tiles_per_cta depend on (E, N, K, sms) only.  If entries is not NULL it receives, per 128-row
+ * weight tile in tile order (E * N / 128 entries, max_entries >= that), six ints: CTA, slot, expert, n-tile, row0, rows. */
+int ob_debug_moe_device_plan(int num_experts, int N, int K, int sms, const int32_t* offsets_host, int total_rows, int* grid,
+                             int* tiles_per_cta, int* entries, int max_entries);
+
 #ifdef __cplusplus
 }
 #endif

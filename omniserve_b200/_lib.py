@@ -115,6 +115,12 @@ _SIGS = {
     "ob_kv4_page_selector": ([C.POINTER(PageSelectorArgs), c_p], c_i),
     "ob_token_streaming_prefill_attention": ([C.POINTER(StreamingPrefillArgs), c_p], c_i),
     "ob_debug_streaming_prefill_plan": ([C.POINTER(StreamingPrefillArgs)] + [c_i] * 3 + [c_p] * 2 + [c_i], c_i),
+    "ob_moe_router_logits": ([c_p] * 3 + [c_i] * 3 + [c_p], c_i),
+    "ob_moe_topk_sort": ([c_p] * 5 + [c_i] * 3 + [c_p], c_i),
+    "ob_moe_expand": ([c_p] * 8 + [c_i] * 3 + [c_p], c_i),
+    "ob_moe_finalize": ([c_p] * 4 + [c_i] * 4 + [c_p], c_i),
+    "ob_w4a8_moe_gemm_dev": ([c_p] * 8 + [c_i] * 5 + [c_p], c_i),
+    "ob_debug_moe_device_plan": ([c_i] * 4 + [c_p, c_i] + [c_p] * 3 + [c_i], c_i),
 }
 EXPORTS = tuple(_SIGS)
 

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, os.environ.get("OB_BUILD_LIBDIR", "lib"))     # e.g. lib_timing for an instrumented variant (OB_LIB_PATH)
 LIB = os.path.join(LIBDIR, "libomniserve_b200.so")
 SOURCES = ["w4a8_gemm.cu", "w4a8_gemm_decode.cu", "w8a8_gemm.cu", "small_ops.cu", "kv4_attention.cu", "lserve_ops.cu", "prefill_attention.cu",
-           "c_api.cu"]
+           "moe_ops.cu", "c_api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--compiler-options", "-fPIC", "-Xptxas", "-v",

@@ -2,6 +2,7 @@
 #include "../../include/omniserve_b200.h"
 #include "kv4_attention.h"
 #include "lserve_ops.h"
+#include "moe_ops.h"
 #include "prefill_attention.h"
 #include "small_ops.h"
 #include "w4a8_gemm.h"
@@ -84,6 +85,48 @@ int ob_w4a8_moe_gemm(const int8_t* in_feats, const int8_t* kernel, const void* w
   if (!in_feats || !kernel || !wscales || !ascales || !w_szs || !a_ssums || !out_feats || !problem_sizes_host) return OB_ERR_ARG;
   return w4a8_moe_gemm_run(in_feats, kernel, H(wscales), H(ascales), H(w_szs), H(a_ssums), HM(out_feats), problem_sizes_host,
                            num_experts, T, N, K, ldc, ST(stream));
+}
+
+int ob_w4a8_moe_gemm_dev(const int8_t* in_feats, const int8_t* kernel, const void* wscales, const void* ascales,
+                         const void* w_szs, const void* a_ssums, void* out_feats, const int32_t* expert_offsets, int num_experts,
+                         int total_rows, int N, int K, int ldc, void* stream) {
+  if (!in_feats || !kernel || !wscales || !ascales || !w_szs || !a_ssums || !out_feats || !expert_offsets) return OB_ERR_ARG;
+  return w4a8_moe_gemm_dev_run(in_feats, kernel, H(wscales), H(ascales), H(w_szs), H(a_ssums), HM(out_feats), expert_offsets,
+                               num_experts, total_rows, N, K, ldc, ST(stream));
+}
+
+int ob_debug_moe_device_plan(int num_experts, int N, int K, int sms, const int32_t* offsets_host, int total_rows, int* grid,
+                             int* tiles_per_cta, int* entries, int max_entries) {
+  return w4a8_moe_dev_plan(num_experts, N, K, sms, offsets_host, total_rows, grid, tiles_per_cta, entries, max_entries);
+}
+
+int ob_moe_router_logits(const void* x, const void* gate_weight, float* logits, int T, int H, int E, void* stream) {
+  if (T > 0 && (!x || !gate_weight || !logits)) return OB_ERR_ARG;
+  return moe_router_logits_run(H(x), H(gate_weight), logits, T, H, E, ST(stream));
+}
+
+int ob_moe_topk_sort(const float* logits, float* routing_weights, int32_t* expert_indices, int32_t* permuted_loc_to_unpermuted_loc,
+                     int32_t* expert_offsets, int T, int E, int k, void* stream) {
+  if (!expert_offsets || (T > 0 && (!logits || !routing_weights || !expert_indices || !permuted_loc_to_unpermuted_loc)))
+    return OB_ERR_ARG;
+  return moe_topk_sort_run(logits, routing_weights, expert_indices, permuted_loc_to_unpermuted_loc, expert_offsets, T, E, k,
+                           ST(stream));
+}
+
+int ob_moe_expand(const int8_t* q_hidden_states, const void* q_input_ssums, const void* q_input_scales,
+                  const int32_t* permuted_loc_to_unpermuted_loc, int8_t* q_out, void* ssums_out, void* scales_out,
+                  int32_t* unpermuted_loc_to_permuted_loc, int T, int k, int H, void* stream) {
+  if (T > 0 && (!q_hidden_states || !q_input_scales || !permuted_loc_to_unpermuted_loc || !q_out || !scales_out ||
+                !unpermuted_loc_to_permuted_loc))
+    return OB_ERR_ARG;
+  return moe_expand_run(q_hidden_states, H(q_input_ssums), H(q_input_scales), permuted_loc_to_unpermuted_loc, q_out, HM(ssums_out),
+                        HM(scales_out), unpermuted_loc_to_permuted_loc, T, k, H, ST(stream));
+}
+
+int ob_moe_finalize(const void* q_w2_out, const float* routing_weights, const int32_t* unpermuted_loc_to_permuted_loc, void* out,
+                    int T, int k, int H, int ldy, void* stream) {
+  if (T > 0 && (!q_w2_out || !routing_weights || !unpermuted_loc_to_permuted_loc || !out)) return OB_ERR_ARG;
+  return moe_finalize_run(H(q_w2_out), routing_weights, unpermuted_loc_to_permuted_loc, HM(out), T, k, H, ldy, ST(stream));
 }
 
 int ob_w8a8_gemm(const int8_t* in_feats, const int8_t* kernel, const void* wscales, const void* ascales, void* out_feats,

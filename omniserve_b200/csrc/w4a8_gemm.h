@@ -45,6 +45,13 @@ int w4a8_gemm_decode_plan(int M, int N, int K, int sms, int ctas_per_sm, int use
 int w4a8_moe_gemm_run(const int8_t* x, const int8_t* qweight, const __half* wscales, const __half* ascales, const __half* w_szs,
                       const __half* a_ssums, __half* out, const int* problem_sizes_host, int num_experts, int T, int N, int K,
                       int ldc, cudaStream_t st);
+// Same GEMM with the expert row ranges in DEVICE memory (offsets [E+1]), at most 64 rows per expert: no host read-back, CUDA-graph
+// capturable.  total_rows = rows of x / out.  w4a8_moe_dev_plan: host-only view of its schedule for an offsets table.
+int w4a8_moe_gemm_dev_run(const int8_t* x, const int8_t* qweight, const __half* wscales, const __half* ascales, const __half* w_szs,
+                          const __half* a_ssums, __half* out, const int* offsets, int num_experts, int total_rows, int N, int K,
+                          int ldc, cudaStream_t st);
+int w4a8_moe_dev_plan(int num_experts, int N, int K, int sms, const int* offsets_host, int total_rows, int* grid, int* tiles_per_cta,
+                      int* entries, int max_entries);
 
 // W8A8 GEMM (w8a8_gemm.cu): out = (in . W^T) * wscales[n] * ascales[m], W plain row-major [N, K] int8.
 int w8a8_gemm_run(const int8_t* in_feats, const int8_t* weight, const __half* wscales, const __half* ascales, __half* out,

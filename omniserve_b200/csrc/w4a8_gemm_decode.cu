@@ -18,6 +18,7 @@
 //
 // Replaces the same reference kernels as w4a8_gemm.cu (per_chn/gemm_cuda.cu:308-657, per_group/gemm_cuda.cu:333-707).
 #include "launch.h"
+#include "moe_ops.h"
 #include "ptx.cuh"
 #include "w4a8_gemm.h"
 
@@ -81,9 +82,19 @@ struct Params {
 // token rows routed to one expert (w4a8_moe_linear.py:83-94: x sorted by expert, `problem_sizes` rows per expert).
 constexpr int MOE_MAX_GROUPS = 64;
 struct MoeTab { int expert[MOE_MAX_GROUPS]; int row0[MOE_MAX_GROUPS]; int rows[MOE_MAX_GROUPS]; };
+// Device-offset grouped mode: slot g is expert g; its rows come from the device table `offsets` [E+1] (moe_slot_rows), read
+// only after griddepcontrol.wait, so the routing of the same decode step can produce it.
+struct MoeDev { const int* offsets; int total_rows; };
 struct NoMoe {};
-template <bool MOE> struct MoeSel { using type = NoMoe; };
-template <> struct MoeSel<true> { using type = MoeTab; };
+template <bool MOE, bool DEV> struct MoeSel { using type = NoMoe; };
+template <> struct MoeSel<true, false> { using type = MoeTab; };
+template <> struct MoeSel<true, true> { using type = MoeDev; };
+OB_DEVICE int moe_expert(const MoeTab& t, int g) { return t.expert[g]; }
+OB_DEVICE int moe_expert(const MoeDev&, int g) { return g; }
+OB_DEVICE void moe_slot(const MoeTab& t, int g, int& row0, int& rows) { row0 = t.row0[g]; rows = t.rows[g]; }
+OB_DEVICE void moe_slot(const MoeDev& d, int g, int& row0, int& rows) {
+  moe_slot_rows(d.offsets[g], d.offsets[g + 1], d.total_rows, &row0, &rows);
+}
 
 struct Seg { int tile, kb0, kb1; };
 
@@ -150,10 +161,10 @@ OB_DEVICE void cluster_reduce_cols(uint32_t stage_u32, uint32_t rank, int row, i
   }
 }
 
-template <int BN, bool PER_GROUP, bool MOE = false>
+template <int BN, bool PER_GROUP, bool MOE = false, bool DEV = false>
 __global__ void __launch_bounds__(NUM_THREADS, 2)
 w4a8_gemm_decode_kernel(const __grid_constant__ CUtensorMap act_map, const __grid_constant__ CUtensorMap w_map, const Params p,
-                        const __grid_constant__ typename MoeSel<MOE>::type moe) {
+                        const __grid_constant__ typename MoeSel<MOE, DEV>::type moe) {
   using C = Cfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -207,7 +218,7 @@ w4a8_gemm_decode_kernel(const __grid_constant__ CUtensorMap act_map, const __gri
         int w_tile = sg.tile;     // row-of-tiles coordinate in the packed weight tensor
         if constexpr (MOE) {
           const int g = sg.tile / p.n_tiles_e;
-          w_tile = moe.expert[g] * p.n_tiles_e + (sg.tile - g * p.n_tiles_e);   // experts are stacked along N
+          w_tile = moe_expert(moe, g) * p.n_tiles_e + (sg.tile - g * p.n_tiles_e);   // experts are stacked along N
         }
         for (int kb = sg.kb0; kb < sg.kb1; kb += KPS) {
           const int cnt = min(KPS, sg.kb1 - kb);
@@ -234,7 +245,11 @@ w4a8_gemm_decode_kernel(const __grid_constant__ CUtensorMap act_map, const __gri
       int stage = 0, phase = 0;
       while (it.next(sg)) {
         int row0 = 0;
-        if constexpr (MOE) row0 = moe.row0[sg.tile / p.n_tiles_e];
+        if constexpr (MOE) {
+          int rows = 0;
+          moe_slot(moe, sg.tile / p.n_tiles_e, row0, rows);
+          if (rows == 0) row0 = 0;   // empty slot: the MMAs still drain the weight ring, nothing is stored
+        }
         for (int kb = sg.kb0; kb < sg.kb1; kb += KPS) {
           const int cnt = min(KPS, sg.kb1 - kb);
           mbar_wait(&ba_empty[stage], phase ^ 1);
@@ -367,9 +382,8 @@ w4a8_gemm_decode_kernel(const __grid_constant__ CUtensorMap act_map, const __gri
       if constexpr (MOE) {
         const int g = sg.tile / p.n_tiles_e;
         nt = sg.tile - g * p.n_tiles_e;
-        m_rows = moe.rows[g];
-        row0 = moe.row0[g];
-        s_off = moe.expert[g] * p.N;
+        moe_slot(moe, g, row0, m_rows);
+        s_off = moe_expert(moe, g) * p.N;
       }
       const int n_row = nt * BM + q * 32 + lane;
       const bool n_ok = n_row < p.N;
@@ -506,10 +520,11 @@ w4a8_gemm_decode_kernel(const __grid_constant__ CUtensorMap act_map, const __gri
   if (warp == 3) OB_GT(30);   // exit
 }
 
-template <int BN>
-static int launch_moe(const CUtensorMap& amap, const CUtensorMap& wmap, const Params& p, const MoeTab& tab, int grid, cudaStream_t st) {
+template <int BN, bool DEV = false>
+static int launch_moe(const CUtensorMap& amap, const CUtensorMap& wmap, const Params& p, const typename MoeSel<true, DEV>::type& tab,
+                      int grid, cudaStream_t st) {
   using C = Cfg<BN>;
-  auto kern = w4a8_gemm_decode_kernel<BN, false, true>;
+  auto kern = w4a8_gemm_decode_kernel<BN, false, true, DEV>;
   static bool attr_done[16] = {};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -523,7 +538,7 @@ static int launch_moe(const CUtensorMap& amap, const CUtensorMap& wmap, const Pa
 template <int BN, bool PG>
 static int launch(const CUtensorMap& amap, const CUtensorMap& wmap, const Params& p, int grid, cudaStream_t st) {
   using C = Cfg<BN>;
-  auto kern = w4a8_gemm_decode_kernel<BN, PG, false>;
+  auto kern = w4a8_gemm_decode_kernel<BN, PG, false, false>;
   static bool attr_done[16] = {};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -544,7 +559,7 @@ static bool cluster_ok(int dev, int s) {
   if (s < 2 || s > 8) return false;
   if (!ok[dev][s]) {
     using C = Cfg<BN>;
-    auto kern = w4a8_gemm_decode_kernel<BN, PG, false>;
+    auto kern = w4a8_gemm_decode_kernel<BN, PG, false, false>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_TOTAL);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(s * 8); cfg.blockDim = dim3(NUM_THREADS); cfg.dynamicSmemBytes = C::SMEM_TOTAL;
@@ -731,6 +746,74 @@ int w4a8_moe_gemm_run(const int8_t* x, const int8_t* qweight, const __half* wsca
     row += problem_sizes_host[e];
   }
   return flush();
+}
+
+// Grouped GEMM with DEVICE-resident row ranges (the decode step of a mixture-of-experts layer, which a CUDA graph replays
+// with a routing it cannot know on the host).  A token routes to k DISTINCT experts, so with <= 64 tokens no expert gets
+// more than one 64-row tile: slot g is statically expert g, the grid and the tiles per CTA depend only on (E, N, K) and the
+// device, and the weight producer streams expert g's tiles before griddepcontrol.wait exactly like the dense decode GEMM.
+// Only row0 / rows of a slot come from `offsets` [E+1] (the routing's expert_offsets), read after the wait by the
+// activation producer and the epilogue; an empty slot streams its weights and stores nothing.  The same whole-K tiles and
+// epilogue as w4a8_moe_gemm_run, so both give bit-identical rows.
+static void moe_dev_schedule(int E, int N, int sms, int* tiles_per_cta, int* grid) {
+  const int n_tiles = E * (N / dec::BM);
+  const int tpc = (n_tiles + 2 * sms - 1) / (2 * sms);   // two CTAs per SM, whole tiles per CTA: no split-K
+  *tiles_per_cta = tpc;
+  *grid = (n_tiles + tpc - 1) / tpc;
+}
+
+int w4a8_moe_gemm_dev_run(const int8_t* x, const int8_t* qweight, const __half* wscales, const __half* ascales, const __half* w_szs,
+                          const __half* a_ssums, __half* out, const int* offsets, int num_experts, int total_rows, int N, int K,
+                          int ldc, cudaStream_t st) {
+  using namespace dec;
+  if (total_rows <= 0) return 0;
+  if (num_experts <= 0 || num_experts > MOE_MAX_GROUPS || N % BM != 0 || K % BK != 0 || ldc < N) return OB_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(qweight) & 15)) return OB_ERR_ALIGN;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 16) return OB_ERR_ARG;
+  const int sms = dev_sms(dev);
+  CUtensorMap amap, wmap;
+  if (int e = make_act_map(&amap, x, total_rows, K, 64)) return e;
+  if (int e = make_w_map(&wmap, qweight, num_experts * N, K, false)) return e;   // experts stacked along N
+  Params p{};
+  p.wscales = wscales; p.ascales = ascales; p.w_szs = w_szs; p.a_ssums = a_ssums; p.out = out;
+  p.ws = nullptr; p.counters = nullptr;   // whole tiles only: no split-K workspace
+  p.M = 64; p.N = N; p.K = K; p.ldc = ldc;
+  p.n_tiles_e = N / BM;
+  p.kb_per_tile = K / BK;
+  p.n_tiles = num_experts * p.n_tiles_e;
+  int tpc = 0, grid = 0;
+  moe_dev_schedule(num_experts, N, sms, &tpc, &grid);
+  p.units_per_cta = tpc * p.kb_per_tile;
+  const MoeDev d{offsets, total_rows};
+  return launch_moe<64, true>(amap, wmap, p, d, grid, st);
+}
+
+// Host-only view of the launch above for a given offsets table (no CUDA call): grid, tiles per CTA and, per tile in tile
+// order, (cta, slot, expert, n-tile, row0, rows) -- the rows after the kernel's clamping (moe_slot_rows).
+int w4a8_moe_dev_plan(int num_experts, int N, int K, int sms, const int* offsets_host, int total_rows, int* grid, int* tiles_per_cta,
+                      int* entries, int max_entries) {
+  using namespace dec;
+  if (num_experts <= 0 || num_experts > MOE_MAX_GROUPS || N <= 0 || N % BM != 0 || K <= 0 || K % BK != 0 || sms <= 0 || total_rows < 0)
+    return OB_ERR_SHAPE;
+  int tpc = 0, g = 0;
+  moe_dev_schedule(num_experts, N, sms, &tpc, &g);
+  if (grid) *grid = g;
+  if (tiles_per_cta) *tiles_per_cta = tpc;
+  if (!entries) return 0;
+  const int n_tiles_e = N / BM, n_tiles = num_experts * n_tiles_e, KB = K / BK;
+  if (!offsets_host || max_entries < n_tiles) return OB_ERR_ARG;
+  const long long upc = (long long)tpc * KB;
+  for (int tile = 0; tile < n_tiles; ++tile) {
+    const int slot = tile / n_tiles_e;
+    int row0 = 0, rows = 0;
+    moe_slot_rows(offsets_host[slot], offsets_host[slot + 1], total_rows, &row0, &rows);
+    int* o = entries + 6 * tile;
+    o[0] = (int)((long long)tile * KB / upc);   // the CTA whose unit range holds the tile (SegIter)
+    o[1] = slot; o[2] = slot; o[3] = tile - slot * n_tiles_e; o[4] = row0; o[5] = rows;
+  }
+  return 0;
 }
 
 }  // namespace ob
